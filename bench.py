@@ -2,12 +2,15 @@
 """bench.py -- CSPN propagation throughput on B200 (contract: see the task brief / DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--algo auto|generic|cluster]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (24-iteration 2D CSPN, '8sum', with sparse depth) over one batch of
 synthetic inputs of BASELINE.json configs[1]: 32 x 1216x352 (W x H) per GPU, fp32.  Weak scaling: every
 rank owns its own 32 images (N=8 is configs[4], 256 images); no data-path collective.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  --dump-outputs DIR also writes what the last timed step returned on rank 0, the
+propagated depth of its 32 images, as DIR/out.npy (float32, 54.8 MB); the inputs are seeded, so two builds can be
+compared output for output.
 """
 import argparse
 import json
@@ -382,7 +385,12 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-other-configs', action='store_true')
     ap.add_argument('--e2e-steps', type=int, default=5)
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the output of the last timed step as DIR/out.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     args.warmup = max(args.warmup, 3)
     quiet_stdout()
 
@@ -446,6 +454,7 @@ def main():
             out = step()
         ev1.record()
         barrier()
+    last_out = out.cpu() if args.dump_outputs and rank == 0 else None
     ms = torch.tensor([ev0.elapsed_time(ev1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -555,6 +564,10 @@ def main():
             line['configs'] = configs
         if gather:
             line['gather'] = gather
+        if last_out is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, 'out.npy'), last_out.numpy().astype(np.float32, copy=False))
         emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -62,6 +62,28 @@ def main():
                         seed=0, B=1, C=1, H=4, W=5, gch=8, sparse='None', n_sample=0)
     print('zero_guidance_nan: all nan =', bool(torch.isnan(out).all()))
     special_cases()
+    port_cases()
+
+
+PORT_SHAPES = [(2, 3, 7, 9), (1, 1, 16, 33)]
+PORT_NORMS = ['8sum', '8sum_abs']
+
+
+def port_name(norm, shape):
+    return f'{norm}_' + 'x'.join(map(str, shape))
+
+
+def port_cases():
+    """tests/golden/port/*.npz: the reference's output for the cases on which the torch-op port must agree with it bit for
+    bit (6 steps, 9 guidance channels, signed sparse depth); inputs travel with the file."""
+    os.makedirs(os.path.join(HERE, 'port'), exist_ok=True)
+    for norm in PORT_NORMS:
+        for shape in PORT_SHAPES:
+            g, d, s = make_inputs(123, *shape, 9, 'signed', 20)
+            out = ref_loader.reference_forward(g, d, s, 6, norm)
+            np.savez_compressed(os.path.join(HERE, 'port', port_name(norm, shape) + '.npz'), guidance=g.numpy(),
+                                blur=d.numpy(), sparse_depth=s.numpy(), out=out.numpy(), prop_time=6, norm_type=norm)
+            print(f'port {port_name(norm, shape)}: absmax={float(out.abs().max()):.4f}')
 
 
 def save_special(name, guidance, blur, sp, n, norm):

@@ -24,7 +24,7 @@ def main():
     import loss as ref_loss
     import utils as ref_utils
     cases = {
-        'nyu_like': (3, (2, 1, 228, 304), 0.0, 1.0),          # dense ground truth
+        'nyu_like': (3, (1, 1, 228, 304), 0.0, 1.0),          # dense ground truth
         'kitti_like': (4, (2, 1, 64, 256), 0.7, 1.0),         # 70 % of the ground truth missing (== 0)
         'close_prediction': (5, (1, 1, 40, 60), 0.2, 0.02),   # errors around the delta thresholds
         'nothing_valid': (6, (1, 1, 8, 8), 1.0, 1.0),

@@ -5,9 +5,12 @@ post_process_layer (torch_resnet_cspn_nyu.py:372-375) and what the model returns
 
     python tests/golden/make_golden_model.py      (build container only: needs /root/reference)
 
-tests/golden/model/nyu_resnet50_tail.npz: guidance (1,8,228,304), blur (1,1,228,304), sparse_depth (1,1,228,304), out.
-The GPU box has no /root/reference: tests/test_reference_model_golden_gpu.py feeds these boundary tensors to the
-B200 module and must reproduce the reference MODEL's output -- the exit criterion of SURVEY.md section 7.2.
+tests/golden/model/nyu_resnet50_tail.npz holds two 80x112 windows of the 228x304 image, at the top-left and the
+bottom-right corner (so every image border is in one of them): guidance_<c> (1,8,80,112), blur_<c> and sparse_depth_<c>
+(1,1,80,112), and out_<c>, the model's output on the part of the window at least `margin` = prop_time + 2 pixels from
+its inner edges.  One step moves information by one pixel, so there the output depends on nothing outside the window.
+tests/test_reference_model_golden_gpu.py feeds these boundary tensors to the B200 module and must reproduce the
+reference MODEL's output -- the exit criterion of SURVEY.md section 7.2.
 float16-rounded storage would break bit-faithfulness of the inputs, so everything is stored as float32 (npz-compressed).
 """
 import importlib
@@ -45,10 +48,23 @@ def main():
         out = net(x)
     os.makedirs(os.path.join(HERE, 'model'), exist_ok=True)
     path = os.path.join(HERE, 'model', 'nyu_resnet50_tail.npz')
-    np.savez_compressed(path, guidance=seen['guidance'].numpy(), blur=seen['blur'].numpy(), sparse_depth=seen['sparse'].numpy(),
-                        out=out.numpy(), prop_time=24, norm_type='8sum')
+    np.savez_compressed(path, **windows(seen['guidance'], seen['blur'], seen['sparse'], out, 24), prop_time=24,
+                        norm_type='8sum')
     print(path, os.path.getsize(path), 'bytes; out absmax', float(out.abs().max()), 'finite', bool(torch.isfinite(out).all()),
           'sparse points', int((seen['sparse'] > 0).sum()))
+
+
+def windows(guidance, blur, sparse, out, prop_time, size=(80, 112)):
+    H, W = out.shape[-2:]
+    m = prop_time + 2
+    rec = dict(image_hw=np.array([H, W]), margin=m)
+    for c, r0, c0 in (('tl', 0, 0), ('br', H - size[0], W - size[1])):
+        win = np.s_[..., r0:r0 + size[0], c0:c0 + size[1]]
+        rec.update({f'guidance_{c}': guidance[win].numpy(), f'blur_{c}': blur[win].numpy(),
+                    f'sparse_depth_{c}': sparse[win].numpy()})
+        valid = np.s_[..., :size[0] - m, :size[1] - m] if c == 'tl' else np.s_[..., m:, m:]
+        rec[f'out_{c}'] = np.ascontiguousarray(out[win].numpy()[valid])
+    return rec
 
 
 if __name__ == '__main__':

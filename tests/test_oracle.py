@@ -1,10 +1,12 @@
-"""CPU tests: the oracle (numpy + C) against the golden vectors produced by the reference module,
-against the reference module itself when /root/reference is mounted, and against each other."""
+"""CPU tests: the oracle (numpy + C) and the torch-op port against the golden vectors produced by the reference
+module, and against each other."""
+import os
+
 import numpy as np
 import pytest
 
-from conftest import golden_names, load_golden
-from oracle import c_oracle, cspn_numpy as onp, ref_loader
+from conftest import GOLDEN_DIR, golden_names, load_golden
+from oracle import c_oracle, cspn_numpy as onp
 
 
 @pytest.mark.parametrize('name', golden_names())
@@ -32,21 +34,19 @@ def test_fp64_spec_bounds_fp32_rounding():
     assert ok and normwise < 1e-6
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='/root/reference not mounted (GPU box)')
 @pytest.mark.parametrize('norm', ['8sum', '8sum_abs'])
 @pytest.mark.parametrize('shape', [(2, 3, 7, 9), (1, 1, 16, 33)])
 def test_oracles_and_torch_port_match_live_reference(norm, shape):
+    """tests/golden/port: inputs and the reference module's output, recorded by tests/golden/make_golden.py."""
     import torch
-    from cspn_b200.synth import make_inputs
     from oracle import cspn_torch_port as tp
-    B, C, H, W = shape
-    g, d, s = make_inputs(123, B, C, H, W, 9, 'signed', 20)
-    ref = ref_loader.reference_forward(g, d, s, 6, norm).numpy()
+    z = np.load(os.path.join(GOLDEN_DIR, 'port', f'{norm}_' + 'x'.join(map(str, shape)) + '.npz'))
+    g, d, s, ref = z['guidance'], z['blur'], z['sparse_depth'], z['out']
+    assert g.shape == (shape[0], 9) + shape[2:] and d.shape == shape and str(z['norm_type']) == norm
     with torch.no_grad():
-        port = tp.cspn2d_torch(g, d, s, 6, norm).numpy()
+        port = tp.cspn2d_torch(torch.from_numpy(g), torch.from_numpy(d), torch.from_numpy(s), 6, norm).numpy()
     assert np.array_equal(port, ref)       # same op sequence -> same bits
-    for out in (onp.cspn2d(g.numpy(), d.numpy(), s.numpy(), 6, norm),
-                c_oracle.cspn2d(g.numpy(), d.numpy(), s.numpy(), 6, norm)):
+    for out in (onp.cspn2d(g, d, s, 6, norm), c_oracle.cspn2d(g, d, s, 6, norm)):
         ok, ratio, _ = onp.parity_ok(out, ref)
         assert ok and ratio < 0.05
 
